@@ -1,9 +1,13 @@
 """Shared helpers of the test-suite: library loaders and the input corpus.
 
 oracle(), ref() and emu() load TEST INFRASTRUCTURE (oracle/, tests/emu); product() loads the
-library under test.  Nothing here reads /root/reference."""
+library under test.  Nothing here reads the reference checkout; reference() and same() let a test compare with the
+reference's own code where oracle/_ref is built and with the digests that code left in tests/golden elsewhere."""
+import atexit
 import functools
+import hashlib
 import importlib
+import json
 import os
 import subprocess
 import sys
@@ -67,6 +71,68 @@ def ref_frontend():
     lib.ref_half_to_float.restype = ctypes.c_float
     lib.ref_half_to_float.argtypes = [ctypes.c_ushort]
     return lib
+
+
+# ---------------------------------------------------------------------------------------------
+# results of the reference's own code: live from oracle/_ref where it is built, else the stored digests
+# ---------------------------------------------------------------------------------------------
+REF_DIGESTS = os.path.join(ROOT, "tests", "golden", "reference_digests.json")
+_RECORD = os.environ.get("ITW_RECORD_REFERENCE")       # set by tests/golden/make_golden_reference.py
+_recorded = {}
+
+
+def digest(a):
+    """dtype, shape and the first 128 bits of the SHA-256 of an array's bytes; -0.0 and 0.0 hash alike, as they compare equal."""
+    a = np.ascontiguousarray(a)
+    if a.dtype.kind == "f":
+        a = a + a.dtype.type(0)
+    return f"{a.dtype.str}{list(a.shape)}:{hashlib.sha256(a.tobytes()).hexdigest()[:32]}"
+
+
+@functools.lru_cache(None)
+def _stored():
+    with open(REF_DIGESTS) as f:
+        return json.load(f)["digests"]
+
+
+def _write_recorded():
+    out = {"generator": "tests/golden/make_golden_reference.py", "digests": {}}
+    if os.path.exists(_RECORD):
+        with open(_RECORD) as f:
+            out = json.load(f)
+    out["digests"].update(_recorded)
+    out["digests"] = dict(sorted(out["digests"].items()))
+    with open(_RECORD, "w") as f:
+        json.dump(out, f, indent=0)
+        f.write("\n")
+
+
+def reference(key, live):
+    """What the reference's own code computes for `key`.  `live` computes it (an array) where the reference build is
+    available and is None elsewhere.  Returns the array when computed live (after checking it against the stored digest,
+    so that the golden file cannot drift from the reference), else the digest stored in tests/golden/reference_digests.json.
+    Compare the result with same()."""
+    if _RECORD:
+        assert live is not None, f"{key}: recording needs the reference build"
+        want = np.ascontiguousarray(live())
+        d = digest(want)
+        assert _recorded.setdefault(key, d) == d, f"{key}: two different results under one key"
+        if len(_recorded) == 1:
+            atexit.register(_write_recorded)
+        return want
+    stored = _stored().get(key)
+    assert stored is not None, f"{key}: no stored reference digest (run tests/golden/make_golden_reference.py)"
+    if live is None:
+        return stored
+    want = np.ascontiguousarray(live())
+    assert digest(want) == stored, f"{key}: the reference build no longer gives the stored result"
+    return want
+
+
+def same(got, want):
+    """got equals a result of reference() in dtype, shape and every element.  Live or stored, the comparison is the same
+    one (by digest), so a test passes with the reference build exactly when it passes without."""
+    return digest(got) == (want if isinstance(want, str) else digest(want))
 
 
 @functools.lru_cache(None)

@@ -138,10 +138,11 @@ def test_gpu_encode_decode_round_trip_full_size():
 
 
 def _ref_decoders():
+    """DirectXTex's own BC1 / BC3 decoder bodies, or None where they are not built."""
     import ctypes
     lib = T.ref_frontend()
     if lib is None:
-        pytest.skip("reference bodies not built (no /root/reference and no prebuilt oracle/_ref)")
+        return None
     for name in ("ref_decode_bc1", "ref_decode_bc3"):
         getattr(lib, name).restype = None
         getattr(lib, name).argtypes = [ctypes.c_void_p, ctypes.c_void_p]
@@ -175,11 +176,8 @@ def test_bc1_bc3_decode_equals_directxtex_decoder_bodies_rounded():
     n = bc1.size // 8
     h = 4 * (n // 64)
     got = e.decode("BC1", bc1[: (h // 4) * 64 * 8], 256, h).reshape(h // 4, 4, 64, 4, 4).transpose(0, 2, 1, 3, 4).reshape(-1, 16, 4)
-    for i in range(got.shape[0]):
-        out = np.zeros(64, np.float32)
-        blk = np.ascontiguousarray(bc1[8 * i:8 * i + 8])
-        lib.ref_decode_bc1(blk.ctypes.data, out.ctypes.data)
-        assert np.array_equal(got[i].astype(np.int64), _rounded(out).reshape(16, 4)), i
+    want = T.reference("bc1_decode_rounded", lib and (lambda: _ref_decode_rounded(lib.ref_decode_bc1, bc1, 8, got.shape[0])))
+    assert T.same(got.astype(np.int64), want), _first_differing(got, want)
     # BC3: colour block always in four-colour mode + every alpha endpoint pair
     blocks = []
     aidx = 0
@@ -194,8 +192,20 @@ def test_bc1_bc3_decode_equals_directxtex_decoder_bodies_rounded():
     bc3 = np.concatenate(blocks)
     h = 4 * (len(blocks) // 64)
     got = e.decode("BC3", bc3, 256, h).reshape(h // 4, 4, 64, 4, 4).transpose(0, 2, 1, 3, 4).reshape(-1, 16, 4)
-    for i in range(got.shape[0]):
-        out = np.zeros(64, np.float32)
-        blk = np.ascontiguousarray(bc3[16 * i:16 * i + 16])
-        lib.ref_decode_bc3(blk.ctypes.data, out.ctypes.data)
-        assert np.array_equal(got[i].astype(np.int64), _rounded(out).reshape(16, 4)), i
+    want = T.reference("bc3_decode_rounded", lib and (lambda: _ref_decode_rounded(lib.ref_decode_bc3, bc3, 16, got.shape[0])))
+    assert T.same(got.astype(np.int64), want), _first_differing(got, want)
+
+
+def _ref_decode_rounded(fn, blocks, bpb, n):
+    """n blocks of `bpb` bytes through a DirectXTex decoder body, rounded like the preview store: (n, 16, 4) int64"""
+    out = np.zeros((n, 64), np.float32)
+    for i in range(n):
+        blk = np.ascontiguousarray(blocks[bpb * i:bpb * i + bpb])
+        fn(blk.ctypes.data, out[i].ctypes.data)
+    return _rounded(out).reshape(n, 16, 4)
+
+
+def _first_differing(got, want):
+    if isinstance(want, str):
+        return "differs from the stored digest of DirectXTex's decode"
+    return int(np.nonzero((got.astype(np.int64) != want).any(axis=(1, 2)))[0][0])

@@ -58,14 +58,14 @@ CASES = [(f, d, p) for f in FAMILIES for d in (8, 16, 32) for p in (1, 2, 3, 4)]
 @pytest.mark.parametrize("fmt,depth,planes", CASES)
 def test_oracle_matches_reference_function_bodies(fmt, depth, planes):
     lib = T.ref_frontend()
-    if lib is None:
-        pytest.skip("reference front end not built (no /root/reference and no prebuilt oracle/_ref)")
     o = T.oracle()
     px = source(depth, planes, 13, 7, seed=depth + planes)
     for flags in flag_sets(fmt, depth, planes):
-        assert np.array_equal(o.convert_pixels(fmt, px, flags), ref_convert(lib, fmt, px, flags)), flags
+        want = T.reference(f"convert:{fmt}:{depth}:{planes}:13x7:{flags}", lib and (lambda: ref_convert(lib, fmt, px, flags)))
+        assert T.same(o.convert_pixels(fmt, px, flags), want), flags
     px = source(depth, planes, 16, 8, seed=3)                       # no padding needed
-    assert np.array_equal(o.convert_pixels(fmt, px, 0), ref_convert(lib, fmt, px, 0))
+    want = T.reference(f"convert:{fmt}:{depth}:{planes}:16x8:0", lib and (lambda: ref_convert(lib, fmt, px, 0)))
+    assert T.same(o.convert_pixels(fmt, px, 0), want)
 
 
 @pytest.mark.parametrize("fmt,depth,planes", CASES)
@@ -90,11 +90,12 @@ def test_half_conversion_is_ieee_where_every_directxmath_version_agrees():
     px = vals.reshape(1, -1, 1)
     got = o.convert_pixels("BC6H", px, 0, pad=False)[0, :, 0]
     assert np.array_equal(got, want)
-    if lib is not None:
-        assert all(lib.ref_float_to_half(float(v)) == int(w) for v, w in zip(vals[:2000], want[:2000]))
-        # half -> float is exact for every normal and denormal half
-        for hbits in list(range(0, 0x7C00, 37)) + [1, 0x3FF, 0x400, 0x7BFF]:
-            assert lib.ref_half_to_float(hbits) == float(np.array([hbits], np.uint16).view(np.float16)[0])
+    ref_halves = T.reference("float_to_half", lib and (lambda: np.array([lib.ref_float_to_half(float(v)) for v in vals[:2000]], np.uint16)))
+    assert T.same(want[:2000], ref_halves)
+    # half -> float is exact for every normal and denormal half
+    hbits = np.array(list(range(0, 0x7C00, 37)) + [1, 0x3FF, 0x400, 0x7BFF], np.uint16)
+    ref_floats = T.reference("half_to_float", lib and (lambda: np.array([lib.ref_half_to_float(int(b)) for b in hbits], np.float32)))
+    assert T.same(hbits.view(np.float16).astype(np.float32), ref_floats)
 
 
 def test_sixteen_bit_rule_is_exact_integer_arithmetic():

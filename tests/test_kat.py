@@ -17,16 +17,22 @@ def solid(v, a=255):
 @pytest.mark.parametrize("which", CPU_APIS)
 def test_bc1_bc3_degenerate_blocks(which):
     api = getattr(T, which)()
-    if api is None:
-        pytest.skip("reference-source build unavailable")
+
+    def check(fmt, v, want_hex, start=0):
+        key = f"kat:{fmt}:solid{v}:{start}"
+        if which == "ref":                         # the reference build, or what it produced where it is not built
+            want = T.reference(key, api and (lambda: api.encode(fmt, solid(v))[start:]))
+            assert T.same(np.frombuffer(bytes.fromhex(want_hex), np.uint8), want), key
+        else:
+            assert api.encode(fmt, solid(v))[start:].tobytes().hex() == want_hex, key
     # all-white: eps-only covariance, both endpoints 0xFFFF, NaN fast_quant -> indices 0 (quirk Q7)
-    assert api.encode("BC1", solid(255)).tobytes().hex() == "ffffffff00000000"
-    assert api.encode("BC1", solid(0)).tobytes().hex() == "0000000000000000"
+    check("BC1", 255, "ffffffff00000000")
+    check("BC1", 0, "0000000000000000")
     # mid grey: c0=127->0x7BEF, c1=128->0x8410, single-colour refine branch (K:424-432)
-    assert api.encode("BC1", solid(128)).tobytes().hex() == "1084108400000000"
+    check("BC1", 128, "1084108400000000")
     # BC3 alpha 255: ep1 = ep0+0.1, q = 0 -> 7 -> 8 -> 1 (K:557-560)
-    assert api.encode("BC3", solid(255)).tobytes().hex() == "ffff499224499224" + "ffffffff00000000"
-    assert api.encode("BC3", solid(128)).tobytes().hex()[16:] == "1084108400000000"
+    check("BC3", 255, "ffff499224499224" + "ffffffff00000000")
+    check("BC3", 128, "1084108400000000", start=8)
 
 
 @pytest.mark.parametrize("which", CPU_APIS)
