@@ -16,7 +16,7 @@ TESTS = os.path.dirname(HERE)
 OUT = os.path.join(HERE, "reference_digests.json")
 CPU_TESTS = ["test_abi.py", "test_bc45_vs_directxtex.py", "test_dds.py", "test_decode.py", "test_decode_vs_directxtex.py",
              "test_frontend.py", "test_kat.py", "test_mips.py", "test_mips_f16.py", "test_oracle_vs_ref.py", "test_random_settings.py",
-             "test_real_content.py", "test_tables.py", "test_gpu_content.py"]
+             "test_real_content.py", "test_tables.py", "test_gpu_content.py", "test_gpu_prepass.py"]
 
 
 def record_gpu_only():
